@@ -365,6 +365,8 @@ def run_ours(args):
     if graph is not None:
         renderer.status()  # raises if a replayed pass overflowed its plan (its results would be void)
         renderer.set_deferred(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs, grads, len(scenes))
     if world > 1:
         t = torch.tensor([elapsed_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -478,6 +480,42 @@ def run_ours(args):
         "clocks": clocks,
     }
     print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, outs, grads, n_views):
+    """Writes what the last timed step returned to its caller - per view the image and z-buffer of the forward and the
+    gradients of the adjoint - as <path>/<name>.npy, flattened, in the float32 / float64 they were computed in.
+    One process only (main() refuses the option otherwise).
+
+    Pixels that no triangle covers have a z of +inf; the z-buffer is written with 0 there and <name>_finite.npy holds
+    1.0 where z is finite, so that every file is finite.  Each output gets an equal share of DUMP_BYTES; a larger one
+    is reduced to the elements at np.sort(np.random.default_rng(0).choice(n, k, replace=False)), the same sample in
+    every run, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {}
+    for v in range(n_views):
+        arrays[f"view{v}_image"] = outs[v]["image"]
+        z = outs[v]["z_buffer"]
+        finite = z.isfinite()
+        arrays[f"view{v}_z_buffer"] = z.where(finite, z.new_zeros(()))
+        arrays[f"view{v}_z_buffer_finite"] = finite.double()  # float64 like z: the same sample of pixels
+        for name in ("ij_b", "colors_b", "uv_b", "shade_b", "texture_b"):
+            if grads[v][name].numel():
+                arrays[f"view{v}_{name}"] = grads[v][name]
+    share = DUMP_BYTES // len(arrays)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().reshape(-1).cpu().numpy()
+        k = share // a.itemsize
+        if a.size > k:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        assert a.dtype in (np.float32, np.float64) and np.isfinite(a).all(), name
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        total += a.nbytes
+    assert total <= DUMP_BYTES, f"dumped {total} bytes"
 
 
 def run_e2e(args, scene, world, dev):
@@ -608,7 +646,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10, help="cap on the e2e (host-buffer) timed steps")
     ap.add_argument("--ref-steps", type=int, default=5, help="cap on the bounded reference-arm repeats")
     ap.add_argument("--cpu-threads", type=int, default=64, help="cap on the reference-arm host threads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (seeded sample of large ones)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        # with N > 1 the shared gradients are all-reduced and cleared on the communication stream inside the step,
+        # so the arrays a caller receives are not left in place after it
+        ap.error("--dump-outputs needs --impl ours in a single process (--gpus 1)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     import __graft_entry__ as entry
 

@@ -6,7 +6,8 @@ Two interchangeable back-ends with the same Python API:
   (C++/DifferentiableRenderer.h ``renderScene`` :2717 / ``renderScene_B`` :2903) compiled by ``oracle/Makefile`` from
   where it lies under /root/reference (never copied into this repository).  ``texfix=True`` selects the variant in
   which the ``=`` of ``bilinear_sample_B`` (DifferentiableRenderer.h:621-624) is patched to ``+=``.
-* ``kind="port"``: ``oracle/liboracle.so`` = our own C restatement (``oracle/deodr_oracle.c``).
+* ``kind="port"``: ``oracle/liboracle.so`` = our own C restatement (``oracle/deodr_oracle.c``).  ``texfix`` is a
+  process-wide switch of that library, so every call of a port oracle sets it to the oracle's own ``texfix`` first.
 
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s ``cpu_baseline`` / ``--impl reference`` legs may
 import this module.  The product package ``deodr_b200`` never does.
@@ -110,6 +111,10 @@ class Oracle:
             C.c_void_p,
         ]
 
+    def _select(self) -> None:
+        if self.kind == "port":
+            self.lib.deodr_oracle_set_texfix(int(self.texfix))
+
     # -- marshalling -------------------------------------------------------------------------------------------
     @staticmethod
     def _pack(scene, with_grads: bool) -> Tuple[SceneC, Dict[str, np.ndarray]]:
@@ -152,6 +157,7 @@ class Oracle:
     # -- API ---------------------------------------------------------------------------------------------------
     def render(self, scene, sigma: float, antialiase_error: bool = False, obs: Optional[np.ndarray] = None):
         """Forward pass -> ``(image[H,W,C], z_buffer[H,W])`` (+ ``err_buffer[H,W]`` in antialiase_error mode)."""
+        self._select()
         s, keep = self._pack(scene, with_grads=False)
         image = np.zeros((s.height, s.width, s.nb_colors))
         z_buffer = np.zeros((s.height, s.width))
@@ -170,6 +176,7 @@ class Oracle:
     def render_b(self, scene, sigma: float, image: np.ndarray, z_buffer: np.ndarray, image_b: np.ndarray,
                  antialiase_error: bool = False, obs=None, err_buffer=None, err_buffer_b=None) -> Dict[str, np.ndarray]:
         """Adjoint pass on COPIES of ``image`` / ``image_b`` -> dict of zero-initialised-then-accumulated gradients."""
+        self._select()
         s, keep = self._pack(scene, with_grads=True)
         image_c = _f64(image).copy()
         z_c = _f64(z_buffer)

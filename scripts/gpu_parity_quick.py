@@ -13,9 +13,7 @@ from deodr_b200.scenes import dense_image_b, soup_scene, torus_scene  # noqa: E4
 from oracle.oracle import Oracle, available  # noqa: E402
 
 tex = np.load(os.path.join(ROOT, "tests/golden/trefle_texture_u8.npy")).astype(np.float64) / 255
-oracle = Oracle("reference", texfix=True) if available("reference", True) else Oracle("port")
-if oracle.kind == "port":
-    oracle.lib.deodr_oracle_set_texfix(1)
+oracle = Oracle("reference", texfix=True) if available("reference", True) else Oracle("port", texfix=True)
 print("oracle:", oracle.kind)
 renderer = Renderer(0)
 

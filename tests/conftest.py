@@ -55,9 +55,7 @@ def checker(build_native):
 
     if available("reference", texfix=True):
         return Oracle("reference", texfix=True)
-    o = Oracle("port")
-    o.lib.deodr_oracle_set_texfix(1)
-    return o
+    return Oracle("port", texfix=True)
 
 
 def load_small(tag):

@@ -1,86 +1,55 @@
-"""TEST INFRASTRUCTURE: runs the REFERENCE package's own tests / examples with deodr_b200 swapped in.
+"""TEST INFRASTRUCTURE: records the renderer calls of the REFERENCE package's own tests / examples.
 
-    python tests/dropin/runner.py <impl> pytest <pytest args ...>     # the reference's test files, unmodified
-    python tests/dropin/runner.py <impl> soup <clockwise 0|1> <antialiase_error 0|1> <iterations>
-    python tests/dropin/runner.py <impl> hand_depth <none|pytorch> <iterations>
-    python tests/dropin/runner.py <impl> hand_rgb <none|pytorch> <iterations>
+    DEODR_STAGED_REFERENCE=<copy of the reference with its Cython extension built> DEODR_RECORD_OUT=<file.npz> \
+    [DEODR_RECORD_CALLS=<forward-call ordinals, comma-separated; all when unset>] \
+    python tests/dropin/runner.py pytest <pytest args ...>     # the reference's test files, unmodified
+    python tests/dropin/runner.py soup <clockwise 0|1> <antialiase_error 0|1> <iterations>
+    python tests/dropin/runner.py hand_depth <none|pytorch> <iterations>
+    python tests/dropin/runner.py hand_rgb <none|pytorch> <iterations>
 
-<impl> = b200: ``sys.modules['deodr.differentiable_renderer_cython']`` is bound to
-``deodr_b200.differentiable_renderer_cython`` BEFORE the reference package is imported - the one-line swap
-INTEGRATION.md describes; nothing else of the staged package (baseline/_ref/deodr: a verbatim, git-ignored copy of
-/root/reference/deodr made by scripts/stage_reference.py) is touched.  <impl> = ref: no swap; needs the reference's own
-Cython extension next to the package (only used in the build container to validate this runner).
-<impl> = ref_noise (build container only, scripts/dropin_sensitivity.py): the reference's own extension with every image
-and gradient it returns multiplied element-wise by 1 + DEODR_NOISE_EPS * N(0, 1) (seed DEODR_NOISE_SEED) - a stand-in
-for fp32 rounding, used to MEASURE how far a perturbation of that size drives the example fits apart.
-Results of the example modes are printed as one JSON line prefixed with RESULT.
+The reference's code runs unchanged with its own extension; ``dropin_calls.Recorder`` wraps the extension's two entry
+points and stores the selected calls with the reference's results (tests/golden/make_dropin_calls.py drives this, and
+tests/test_dropin_reference.py replays the result through deodr_b200).
 """
-import json
+import atexit
 import os
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(os.path.dirname(HERE))
-STAGED = os.environ.get("DEODR_STAGED_REFERENCE", os.path.join(ROOT, "baseline", "_ref"))
 
 
 def main():
-    impl, mode, args = sys.argv[1], sys.argv[2], sys.argv[3:]
-    sys.path[:0] = [os.path.join(HERE, "stubs"), STAGED, ROOT]
+    mode, args = sys.argv[1], sys.argv[2:]
+    staged = os.environ["DEODR_STAGED_REFERENCE"]
+    sys.path[:0] = [os.path.join(HERE, "stubs"), staged]
     import cv2
 
     cv2.waitKey = lambda *a, **k: -1
     cv2.imshow = lambda *a, **k: None
-    if impl == "b200":
-        import deodr_b200.differentiable_renderer_cython as shim
-
-        sys.modules["deodr.differentiable_renderer_cython"] = shim
     import deodr  # the staged reference package
+    from deodr import differentiable_renderer_cython as ffi
+    from dropin_calls import Recorder
 
-    assert os.path.abspath(deodr.__file__).startswith(os.path.abspath(STAGED)), deodr.__file__
-    if impl == "b200":
-        from deodr import differentiable_renderer_cython as bound
-
-        assert bound.__name__ == "deodr_b200.differentiable_renderer_cython", bound.__name__
-    if impl == "ref_noise":
-        import numpy as np
-        from deodr import differentiable_renderer_cython as ffi
-
-        rng = np.random.default_rng(int(os.environ.get("DEODR_NOISE_SEED", "0")))
-        eps = float(os.environ.get("DEODR_NOISE_EPS", "1e-7"))
-        fwd, bwd = ffi.renderSceneCpp, ffi.renderSceneBCpp
-
-        def noisy(a):
-            a *= 1.0 + eps * rng.standard_normal(a.shape)
-
-        def render(scene, sigma, image, z_buffer, *a, **k):
-            fwd(scene, sigma, image, z_buffer, *a, **k)
-            noisy(image)
-
-        def render_b(scene, *a, **k):
-            bwd(scene, *a, **k)
-            for name in ("ij_b", "colors_b", "uv_b", "shade_b", "texture_b"):
-                noisy(getattr(scene, name))
-
-        ffi.renderSceneCpp, ffi.renderSceneBCpp = render, render_b
+    assert os.path.abspath(deodr.__file__).startswith(os.path.abspath(staged)), deodr.__file__
+    keep = os.environ.get("DEODR_RECORD_CALLS")
+    rec = Recorder(ffi.renderSceneCpp, ffi.renderSceneBCpp, None if not keep else {int(i) for i in keep.split(",")})
+    ffi.renderSceneCpp, ffi.renderSceneBCpp = rec.render, rec.render_b
+    atexit.register(rec.save, os.environ["DEODR_RECORD_OUT"])
     if mode == "pytest":
         import pytest
 
-        sys.exit(pytest.main(["-q", "-x", "-p", "no:cacheprovider", "--rootdir", STAGED] + args))
+        sys.exit(pytest.main(["-q", "-x", "-p", "no:cacheprovider", "--rootdir", staged] + args))
     if mode == "soup":
         from deodr.examples.triangle_soup_fitting import run
 
-        losses, hashes = run(nb_max_iter=int(args[2]), display=False, clockwise=bool(int(args[0])),
-                             antialiase_error=bool(int(args[1])))
-        print("RESULT " + json.dumps({"losses": losses, "hashes": hashes}))
+        run(nb_max_iter=int(args[2]), display=False, clockwise=bool(int(args[0])), antialiase_error=bool(int(args[1])))
         return
     if mode in ("hand_depth", "hand_rgb"):
         if mode == "hand_depth":
             from deodr.examples.depth_image_hand_fitting import run
         else:
             from deodr.examples.rgb_image_hand_fitting import run
-        energies = run(dl_library=args[0], plot_curves=False, display=False, save_images=False, max_iter=int(args[1]))
-        print("RESULT " + json.dumps({"energies": [float(e) for e in energies]}))
+        run(dl_library=args[0], plot_curves=False, display=False, save_images=False, max_iter=int(args[1]))
         return
     raise SystemExit(f"unknown mode {mode}")
 

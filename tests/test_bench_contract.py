@@ -53,3 +53,13 @@ def test_reference_arm_line(build_native):
     assert line["cpu_baseline"]["value"] == line["value"] == line["e2e"]["value"]
     assert line["e2e"]["h2d_bytes_per_step"] == 0 == line["e2e"]["d2h_bytes_per_step"]
     assert line["config"]["workload"].startswith("c2")
+
+
+def test_dump_outputs_refused_beyond_one_process(tmp_path):
+    """The shared gradients of a multi-process step are cleared after their all-reduce: nothing to dump there."""
+    dump = tmp_path / "dump"
+    for extra, env in ((["--impl", "reference"], {}), ([], {"WORLD_SIZE": "2"})):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(dump), *extra],
+                             capture_output=True, text=True, timeout=120, env=dict(os.environ, **env))
+        assert out.returncode == 2 and "--dump-outputs needs" in out.stderr, out.stderr
+        assert not dump.exists()

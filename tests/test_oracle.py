@@ -9,6 +9,7 @@ import pytest
 from conftest import GOLDEN, SMALL_TAGS, load_small
 
 from deodr_b200.scenes import dense_image_b, soup_scene, torus_scene
+from oracle.oracle import Oracle
 
 sha = lambda a: hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()  # noqa: E731
 
@@ -76,11 +77,7 @@ def test_port_matches_golden_small(tag, port_oracle):
     image, z = port_oracle.render(scene, float(d["sigma"]))
     assert np.array_equal(image, d["image"]) and np.array_equal(z, d["z"])
     if "ij_b" in d:
-        port_oracle.lib.deodr_oracle_set_texfix(1)
-        try:
-            g = port_oracle.render_b(scene, float(d["sigma"]), image, z, dense_image_b(image))
-        finally:
-            port_oracle.lib.deodr_oracle_set_texfix(0)
+        g = Oracle("port", texfix=True).render_b(scene, float(d["sigma"]), image, z, dense_image_b(image))
         for name in ("ij_b", "colors_b", "uv_b", "shade_b"):
             assert np.array_equal(g[name], d[name]), name
         assert np.array_equal(g["texture_b"].astype(np.float32), d["texture_b"])
