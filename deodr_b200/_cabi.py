@@ -161,6 +161,9 @@ SYMBOLS = [
      [C.c_void_p, C.c_int, C.POINTER(SceneView), C.POINTER(ViewIO), C.c_double, C.c_int, C.c_void_p]),
     ("deodr_b200_render_b_views", C.c_int,
      [C.c_void_p, C.c_int, C.POINTER(SceneView), C.POINTER(ViewIO), C.POINTER(Grads), C.c_double, C.c_int, C.c_void_p]),
+    ("deodr_b200_render_b_views_depths", C.c_int,
+     [C.c_void_p, C.c_int, C.POINTER(SceneView), C.POINTER(ViewIO), C.POINTER(Grads), C.POINTER(C.c_void_p), C.c_double,
+      C.c_int, C.c_void_p]),
     ("deodr_b200_workspace_set_deferred", C.c_int, [C.c_void_p, C.c_int]),
     ("deodr_b200_workspace_status", C.c_int, [C.c_void_p]),
     ("deodr_b200_view_generation", C.c_int64, [C.c_void_p, C.c_int]),

@@ -512,7 +512,8 @@ static bool stream_is_capturing(cudaStream_t st) {
     return status != cudaStreamCaptureStatusNone;
 }
 
-static int validate_view(const DeodrSceneView *v, bool backward) {
+// persp_adjoint: the caller is the entry point that has the perspective-correct adjoint (deodr_b200_render_b_views_depths)
+static int validate_view(const DeodrSceneView *v, bool backward, bool persp_adjoint = false) {
     if (!v) return set_error(DEODR_B200_EINVAL, "scene == NULL");
     // zero-sized arrays may legitimately come with a null data pointer
     const bool tris = v->nb_triangles > 0, verts = v->nb_vertices > 0;
@@ -540,7 +541,7 @@ static int validate_view(const DeodrSceneView *v, bool backward) {
         if (!v->backface_culling)
             return set_error(DEODR_B200_EUNSUPPORTED,
                              "You have to use backface_culling true if you ant to compute gradients");
-        if (v->perspective_correct)
+        if (v->perspective_correct && !persp_adjoint)
             return set_error(DEODR_B200_EUNSUPPORTED,
                              "backward gradient propagation not supported yet with perspective_correct=True");
     }
@@ -1166,8 +1167,11 @@ static int render_views_impl(DeodrWorkspace *ws, int n_views, const DeodrSceneVi
     return DEODR_B200_OK;
 }
 
+// depths_b: per-view [V] fp32 device pointers (or NULL entries) of deodr_b200_render_b_views_depths; NULL for the entry
+// points without the perspective-correct adjoint.
 static int render_b_views_impl(DeodrWorkspace *ws, int n_views, const DeodrSceneView *views, const DeodrViewIO *io,
-                               const DeodrGrads *grads, double sigma, int flags, void *stream) {
+                               const DeodrGrads *grads, float *const *depths_b, bool persp_adjoint, double sigma,
+                               int flags, void *stream) {
     if (!ws) return set_error(DEODR_B200_EINVAL, "ws == NULL");
     if (n_views < 0 || (n_views > 0 && (!views || !io || !grads))) return set_error(DEODR_B200_EINVAL, "bad view list");
     const bool err_mode = (flags & DEODR_B200_ANTIALIASE_ERROR) != 0;
@@ -1175,7 +1179,10 @@ static int render_b_views_impl(DeodrWorkspace *ws, int n_views, const DeodrScene
     CUDA_TRY(cudaSetDevice(ws->device));
     const bool capturing = stream_is_capturing(st);
     for (int i = 0; i < n_views; i++) {
-        if (int rc = validate_view(&views[i], true)) return rc;
+        if (int rc = validate_view(&views[i], true, persp_adjoint)) return rc;
+        if (err_mode && views[i].perspective_correct)
+            return set_error(DEODR_B200_EUNSUPPORTED,
+                             "antialiase_error has no adjoint with perspective_correct=True");
         const DeodrViewIO &o = io[i];
         if (!o.z_buffer || !o.owner) return set_error(DEODR_B200_EINVAL, "z_buffer / owner is NULL");
         if (err_mode) {
@@ -1207,7 +1214,9 @@ static int render_b_views_impl(DeodrWorkspace *ws, int n_views, const DeodrScene
     for (int i = 0; i < n_views; i++) {  // accumulators (not while capturing: a warm-up pass has sized them)
         ViewSlot *v = ws->slots[i];
         if (v->plan.cap_edges > 0) {
-            const size_t need = (size_t)v->plan.cap_edges * edge_acc_stride(views[i].nb_colors) * sizeof(double);
+            SceneView sv;
+            memcpy(&sv, &views[i], sizeof(sv));
+            const size_t need = (size_t)v->plan.cap_edges * deodr_edge_acc_stride(sv) * sizeof(double);
             if (need > v->edge_acc.bytes) {
                 if (capturing) return set_error(DEODR_B200_EINVAL, "stream capture needs a warm-up pass outside the capture");
                 if (v->edge_acc.ensure(need, &ws->bytes)) return DEODR_B200_ECUDA;
@@ -1220,7 +1229,8 @@ static int render_b_views_impl(DeodrWorkspace *ws, int n_views, const DeodrScene
         for (int i = 0; i < n_views; i++) {
             SceneView s;
             memcpy(&s, &views[i], sizeof(s));
-            deodr_launch_backward(ws, ws->slots[i], ws->lanes[i % used], s, io[i], sigma, flags, grads[i]);
+            deodr_launch_backward(ws, ws->slots[i], ws->lanes[i % used], s, io[i], sigma, flags, grads[i],
+                                  depths_b ? depths_b[i] : nullptr);
         }
         close_lanes(ws, st, used);
         CUDA_TRY(cudaGetLastError());
@@ -1235,6 +1245,7 @@ static int render_b_views_impl(DeodrWorkspace *ws, int n_views, const DeodrScene
             key.put(views[i]);
             key.put(io[i]);
             key.put(grads[i]);
+            key.put(depths_b ? depths_b[i] : nullptr);
             put_slot(&key, ws->slots[i]);
         }
         const int rc = launch_cached(ws, &ws->bwd_graph, key, st, enqueue_all);
@@ -1450,7 +1461,14 @@ int deodr_b200_render_views(DeodrWorkspace *ws, int n_views, const DeodrSceneVie
 
 int deodr_b200_render_b_views(DeodrWorkspace *ws, int n_views, const DeodrSceneView *views, const DeodrViewIO *io,
                               const DeodrGrads *grads, double sigma, int flags, void *stream) {
-    return render_b_views_impl(ws, n_views, views, io, grads, sigma, flags, stream);
+    return render_b_views_impl(ws, n_views, views, io, grads, nullptr, false, sigma, flags, stream);
+}
+
+int deodr_b200_render_b_views_depths(DeodrWorkspace *ws, int n_views, const DeodrSceneView *views,
+                                     const DeodrViewIO *io, const DeodrGrads *grads, float *const *depths_b,
+                                     double sigma, int flags, void *stream) {
+    if (n_views > 0 && !depths_b) return set_error(DEODR_B200_EINVAL, "depths_b == NULL (pass an array of NULLs)");
+    return render_b_views_impl(ws, n_views, views, io, grads, depths_b, true, sigma, flags, stream);
 }
 
 int deodr_b200_render(DeodrWorkspace *ws, const DeodrSceneView *scene, double sigma, float *image, double *z_buffer,
@@ -1472,7 +1490,7 @@ int deodr_b200_render_b(DeodrWorkspace *ws, const DeodrSceneView *scene, double 
     io.z_buffer = const_cast<double *>(z_buffer);
     io.owner = const_cast<int32_t *>(owner);
     io.image_b = image_b;
-    return render_b_views_impl(ws, 1, scene, &io, grads, sigma, 0, stream);
+    return render_b_views_impl(ws, 1, scene, &io, grads, nullptr, false, sigma, 0, stream);
 }
 
 }  // extern "C"

@@ -3,7 +3,8 @@
 //   k_interior_bwd                        (aux)  pixels of large triangles elsewhere
 //   k_small_tri_bwd                              triangle-parallel adjoint of the small triangles
 // Everything strides over device-side counts left by the forward pass of the same view slot (kernels.cu); a forward
-// that overflowed its plan makes these kernels return at once (nothing is accumulated).
+// that overflowed its plan makes these kernels return at once (nothing is accumulated).  The perspective-correct
+// instances (PERSP) run the same phases with pixel_adjoint_persp and the edge layout of edge_acc_stride_persp.
 #include <cstdlib>
 #include <cstring>
 
@@ -24,16 +25,19 @@ __global__ void k_error_image_b(const float *image, const float *obs, const floa
 // what is left of their colour adjoint.  ERR: the antialiase_error variant (DR.h:2296-2336, 2542-2576); compat = the
 // reference's dropped row term reproduced (phase_edge_adjoint_error).
 // (register budgets are pinned: the allocator's own choice moved 64 -> 80 on an unrelated signature change)
-template <int MAXC, bool TEX, bool ERR>
+// PERSP: perspective_correct as a compile-time constant (instances with ERR = false only; depths_b is written by them).
+template <int MAXC, bool TEX, bool ERR, bool PERSP>
 __global__ void __launch_bounds__(EDGE_NT, DEODR_EDGE_MIN_CTAS) k_raster_bwd(SceneView s, double sigma, TileDiv tiles_x, EdgeTiles et,
                                                    const uint32_t *span_cache, TieTable ties,
                                                    const double *z_buffer,
                                                    const int *owner, const float *image_b, const float *obs,
                                                    const float *err_b, int compat, DeodrGrads grads,
-                                                   double *edge_acc, const __grid_constant__ FrameMaps maps) {
+                                                   double *edge_acc, const __grid_constant__ FrameMaps maps,
+                                                   float *depths_b) {
+    static_assert(!(ERR && PERSP), "antialiase_error has no perspective-correct adjoint");
     if (et.scal[SC_OVERFLOW]) return;
     fix_channel_count<MAXC, TEX>(s);
-    s.perspective_correct = 0;  // the adjoint is only defined without it (validate_view rejects it): folds the branches
+    s.perspective_correct = PERSP ? 1 : 0;  // folds the branches
     __shared__ TileShared sh;
     // the tile's image_b / owner / z-buffer blocks arrive as three TMA tile loads (UTMALDG) issued by one thread
     __shared__ alignas(128) float t_img[MAXC <= 4 ? NT * MAXC : 4];
@@ -141,22 +145,23 @@ __global__ void __launch_bounds__(EDGE_NT, DEODR_EDGE_MIN_CTAS) k_raster_bwd(Sce
         }
         // a pixel overdrawn by edges in error mode: its colour adjoint comes from what is left of the residual's
         if (ERR && inside && ea.has) residual_adjoint<MAXC>(s, ea.col, obs_px, ea.g, a.g);
-        interior_adjoint_warp<MAXC>(s, x, y, inside && p.bown >= 0, p, a.g, grads);
+        interior_adjoint_warp<MAXC>(s, x, y, inside && p.bown >= 0, p, a.g, grads, depths_b);
     }
 }
 
 // Interior adjoint of the pixels owned by LARGE triangles in the tiles without silhouette edges: no shared memory, no
 // z-buffer read; the gradients are summed per owner inside each warp before the scatter (interior_adjoint_warp).
-template <int MAXC, bool TEX>
+template <int MAXC, bool TEX, bool PERSP>
 #ifndef DEODR_INTERIOR_MIN_CTAS
 #define DEODR_INTERIOR_MIN_CTAS 3  // 85 registers: 39.2 us vs 40.3 us at 64 and 47.6 us at 51 (measured, c5)
 #endif
 __global__ void __launch_bounds__(NT, DEODR_INTERIOR_MIN_CTAS) k_interior_bwd(SceneView s, TileDiv tiles_x, const int *large_tiles,
                                                      const int *scal, const int *edge_cursor, TieTable ties,
-                                                     const int *owner, const float *image_b, DeodrGrads grads) {
+                                                     const int *owner, const float *image_b, DeodrGrads grads,
+                                                     float *depths_b) {
     if (scal[SC_OVERFLOW]) return;
     fix_channel_count<MAXC, TEX>(s);
-    s.perspective_correct = 0;  // the adjoint is only defined without it (validate_view rejects it): folds the branches
+    s.perspective_correct = PERSP ? 1 : 0;  // folds the branches
     const int tid = threadIdx.x, total = scal[SC_LARGE_TILES];
     for (int b = blockIdx.x; b < total; b += gridDim.x) {  // one CTA per tile with large triangles binned
         const int tile_id = large_tiles[b];
@@ -165,7 +170,7 @@ __global__ void __launch_bounds__(NT, DEODR_INTERIOR_MIN_CTAS) k_interior_bwd(Sc
         const int x = tile.x0 + tid % TS, y = tile.y0 + tid / TS;
         const bool inside = x < s.width && y < s.height;
         PixelState<MAXC> p;
-        p.z = 0.0;  // only read by the perspective-correct forward path
+        p.z = 0.0;  // only read by the perspective-correct forward path (the adjoint recomputes the pixel's depth)
         p.own = p.bown = -1;
         float g[MAXC];
         if (inside) {
@@ -175,27 +180,27 @@ __global__ void __launch_bounds__(NT, DEODR_INTERIOR_MIN_CTAS) k_interior_bwd(Sc
             if (p.bown >= 0)
                 for (int k = 0; k < s.nb_colors; k++) g[k] = image_b[idx * s.nb_colors + k];
         }
-        interior_adjoint_warp<MAXC>(s, x, y, inside && p.bown >= 0, p, g, grads);
+        interior_adjoint_warp<MAXC>(s, x, y, inside && p.bown >= 0, p, g, grads, depths_b);
     }
 }
 
 // Triangle-parallel interior adjoint of the small triangles (one thread per entry of the compacted small list).
-template <int MAXC, bool TEX>
+template <int MAXC, bool TEX, bool PERSP>
 #ifndef DEODR_SMALL_MIN_CTAS
 #define DEODR_SMALL_MIN_CTAS 8
 #endif
 __global__ void __launch_bounds__(128, DEODR_SMALL_MIN_CTAS) k_small_tri_bwd(SceneView s, int tiles_x, const int *small_ids, const int *scal,
                                                        const int *edge_cursor, TieTable ties, const int *owner,
-                                                       const float *image_b, DeodrGrads grads) {
+                                                       const float *image_b, DeodrGrads grads, float *depths_b) {
     if (scal[SC_OVERFLOW]) return;
     fix_channel_count<MAXC, TEX>(s);
-    s.perspective_correct = 0;  // the adjoint is only defined without it (validate_view rejects it): folds the branches
+    s.perspective_correct = PERSP ? 1 : 0;  // folds the branches
     // one thread per entry (no stride loop: its registers cost this kernel its occupancy); the launch covers the exact
     // count when the forward's verdict has been read, every triangle otherwise
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= scal[SC_SMALL]) return;
     small_triangle_adjoint<MAXC, DevEnv>(s, small_ids[i], tiles_x, edge_cursor, owner, ties.pairs, image_b, grads.ij_b,
-                                         grads.colors_b, grads.uv_b, grads.shade_b, grads.texture_b);
+                                         grads.colors_b, grads.uv_b, grads.shade_b, grads.texture_b, depths_b);
 }
 
 // Record-parallel interior adjoint of the small triangles (small_record_adjoint, phases.h; opt-in, see launch_bwd for the
@@ -219,7 +224,7 @@ __global__ void __launch_bounds__(128, DEODR_SMALL_MIN_CTAS) k_small_rec_bwd(Sce
                                                        const __grid_constant__ FrameMaps maps) {
     if (scal[SC_OVERFLOW]) return;
     fix_channel_count<MAXC, TEX>(s);
-    s.perspective_correct = 0;  // the adjoint is only defined without it (validate_view rejects it): folds the branches
+    s.perspective_correct = 0;  // perspective-correct views take k_small_tri_bwd (launch_bwd): folds the branches
     const int tile_id = blockIdx.x, tid = threadIdx.x;
     const int n = segment_size(seg, tile_id);
     if (n == 0) return;
@@ -261,18 +266,26 @@ __global__ void __launch_bounds__(128, DEODR_SMALL_MIN_CTAS) k_small_rec_bwd(Sce
     }
 }
 
+template <bool PERSP>
 __global__ void k_finalize_edges(SceneView s, EdgeList edges, const int *scal, double sigma, const double *edge_acc,
-                                 DeodrGrads grads) {
+                                 DeodrGrads grads, float *depths_b) {
     if (scal[SC_OVERFLOW]) return;
+    s.perspective_correct = PERSP ? 1 : 0;
+    const int stride = PERSP ? edge_acc_stride_persp(s.nb_colors) : edge_acc_stride(s.nb_colors);
     const int n = min(*edges.count, edges.capacity);
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
-        finalize_edge<DevEnv>(s, edges.ids[i], sigma, edge_acc + (size_t)i * edge_acc_stride(s.nb_colors), grads.ij_b,
-                              grads.colors_b, grads.uv_b, grads.shade_b);
+        finalize_edge<DevEnv>(s, edges.ids[i], sigma, edge_acc + (size_t)i * stride, grads.ij_b, grads.colors_b,
+                              grads.uv_b, grads.shade_b, depths_b);
 }
 
-template <int MAXC>
+// Rows of the per-edge accumulators of a view (the perspective-correct instances use their own layout).
+int deodr_edge_acc_stride(const SceneView &s) {
+    return s.perspective_correct ? edge_acc_stride_persp(s.nb_colors) : edge_acc_stride(s.nb_colors);
+}
+
+template <int MAXC, bool PERSP>
 static void launch_bwd(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneView &s, const DeodrViewIO &io,
-                       double sigma, int flags, const DeodrGrads &g) {
+                       double sigma, int flags, const DeodrGrads &g, float *depths_b) {
     // Three independent chains (disjoint pixel sets, all accumulate with atomics): edge tiles (longest tail: launched
     // first so that its CTAs are dispatched first), tiles with large triangles, small triangles.
     cudaStream_t st = lane.main;
@@ -304,21 +317,22 @@ static void launch_bwd(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneV
               encode_tile_map(&maps.z, io.z_buffer, 8, false, s.height, s.width, TS, TS);
     if (edges) {
         cudaStream_t se = fork_stream(ws, lane, 1, &first);
-        cudaMemsetAsync(v->edge_acc.ptr, 0, (size_t)plan.cap_edges * edge_acc_stride(C) * sizeof(double), se);
+        cudaMemsetAsync(v->edge_acc.ptr, 0, (size_t)plan.cap_edges * deodr_edge_acc_stride(s) * sizeof(double), se);
         const EdgeTiles et = edge_tiles_of(v);
         const int grid = at_least_one(v->hints_exact && !ws->capturing_internally ? plan.hint_edge_tiles : plan.cap_edge_tiles);
         {
             PhaseTimer timer(ws, DEODR_B200_PH_EDGE_BWD, se);
-#define DEODR_RASTER_BWD(X, R) k_raster_bwd<MAXC, X, R><<<grid, EDGE_NT, 0, se>>>(s, sigma, div, et, v->edge_spans.as<uint32_t>(), ties, io.z_buffer, io.owner, image_b, io.obs, io.err_buffer_b, compat, g, v->edge_acc.as<double>(), maps)
-            if (tex) { if (err_mode) DEODR_RASTER_BWD(true, true); else DEODR_RASTER_BWD(true, false); }
+#define DEODR_RASTER_BWD(X, R) k_raster_bwd<MAXC, X, R, PERSP && !R><<<grid, EDGE_NT, 0, se>>>(s, sigma, div, et, v->edge_spans.as<uint32_t>(), ties, io.z_buffer, io.owner, image_b, io.obs, io.err_buffer_b, compat, g, v->edge_acc.as<double>(), maps, depths_b)
+            if (PERSP) { if (tex) DEODR_RASTER_BWD(true, false); else DEODR_RASTER_BWD(false, false); }  // (no ERR)
+            else if (tex) { if (err_mode) DEODR_RASTER_BWD(true, true); else DEODR_RASTER_BWD(true, false); }
             else     { if (err_mode) DEODR_RASTER_BWD(false, true); else DEODR_RASTER_BWD(false, false); }
 #undef DEODR_RASTER_BWD
         }
         {
             PhaseTimer timer(ws, DEODR_B200_PH_EDGE_FINALIZE, se);
             const EdgeList el{v->scal + SC_EDGES, v->edge_ids.as<int>(), v->edge_keys.as<uint64_t>(), plan.cap_edges};
-            k_finalize_edges<<<at_least_one(grid_for(plan.hint_edges, 128)), 128, 0, se>>>(s, el, v->scal, sigma,
-                                                                                           v->edge_acc.as<double>(), g);
+            k_finalize_edges<PERSP><<<at_least_one(grid_for(plan.hint_edges, 128)), 128, 0, se>>>(
+                s, el, v->scal, sigma, v->edge_acc.as<double>(), g, depths_b);
         }
         ws->launches += 2;
     }
@@ -327,8 +341,8 @@ static void launch_bwd(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneV
         cudaStream_t sl = fork_stream(ws, lane, 2, &first);
         PhaseTimer timer(ws, DEODR_B200_PH_INTERIOR_BWD, sl);
         const int grid = at_least_one(plan.hint_large_tiles < v->num_tiles ? plan.hint_large_tiles : v->num_tiles);
-        (tex ? k_interior_bwd<MAXC, true> : k_interior_bwd<MAXC, false>)<<<grid, NT, 0, sl>>>(
-            s, div, v->large_tiles.as<int>(), v->scal, edge_cursor, ties, io.owner, image_b, g);
+        (tex ? k_interior_bwd<MAXC, true, PERSP> : k_interior_bwd<MAXC, false, PERSP>)<<<grid, NT, 0, sl>>>(
+            s, div, v->large_tiles.as<int>(), v->scal, edge_cursor, ties, io.owner, image_b, g, depths_b);
         ws->launches++;
     }
     {
@@ -338,10 +352,11 @@ static void launch_bwd(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneV
         // vertex gathers and the fifteen atomics per thread are what it costs, not the bounding-box reads, and 1.7x
         // more threads pay them - and k_interior_bwd beside it slows from 61 to 73 us); 16 renders of 200k triangles at
         // 512^2: 0.723 vs 0.695 ms; 1M textured triangles: 0.621 vs 0.632 ms.
-        if (!ws->small_by_record) {  // (read from the environment when the workspace is created)
+        // Perspective-correct views always take the triangle-parallel form (k_small_rec_bwd has no PERSP instance).
+        if (!ws->small_by_record || PERSP) {  // (read from the environment when the workspace is created)
             const int entries = v->hints_exact && !ws->capturing_internally ? plan.hint_small : s.nb_triangles;
-            (tex ? k_small_tri_bwd<MAXC, true> : k_small_tri_bwd<MAXC, false>)<<<at_least_one(grid_for(entries, 128)), 128, 0, st>>>(
-                s, v->tiles_x, v->small_ids.as<int>(), v->scal, edge_cursor, ties, io.owner, image_b, g);
+            (tex ? k_small_tri_bwd<MAXC, true, PERSP> : k_small_tri_bwd<MAXC, false, PERSP>)<<<at_least_one(grid_for(entries, 128)), 128, 0, st>>>(
+                s, v->tiles_x, v->small_ids.as<int>(), v->scal, edge_cursor, ties, io.owner, image_b, g, depths_b);
         } else {
             const TileSegments seg{v->small_offset.as<int>(), v->small_cursor};
             (tex ? k_small_rec_bwd<MAXC, true> : k_small_rec_bwd<MAXC, false>)<<<v->num_tiles, 128, 0, st>>>(
@@ -354,11 +369,18 @@ static void launch_bwd(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneV
 }
 
 
-void deodr_launch_backward(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneView &s, const DeodrViewIO &io,
-                           double sigma, int flags, const DeodrGrads &g) {
+template <bool PERSP>
+static void launch_bwd_channels(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneView &s, const DeodrViewIO &io,
+                                double sigma, int flags, const DeodrGrads &g, float *depths_b) {
     const int C = s.nb_colors;
-    if (C == 1) launch_bwd<1>(ws, v, lane, s, io, sigma, flags, g);
-    else if (C == 3) launch_bwd<3>(ws, v, lane, s, io, sigma, flags, g);
-    else if (C <= 4) launch_bwd<4>(ws, v, lane, s, io, sigma, flags, g);
-    else launch_bwd<16>(ws, v, lane, s, io, sigma, flags, g);
+    if (C == 1) launch_bwd<1, PERSP>(ws, v, lane, s, io, sigma, flags, g, depths_b);
+    else if (C == 3) launch_bwd<3, PERSP>(ws, v, lane, s, io, sigma, flags, g, depths_b);
+    else if (C <= 4) launch_bwd<4, PERSP>(ws, v, lane, s, io, sigma, flags, g, depths_b);
+    else launch_bwd<16, PERSP>(ws, v, lane, s, io, sigma, flags, g, depths_b);
+}
+
+void deodr_launch_backward(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneView &s, const DeodrViewIO &io,
+                           double sigma, int flags, const DeodrGrads &g, float *depths_b) {
+    if (s.perspective_correct) launch_bwd_channels<true>(ws, v, lane, s, io, sigma, flags, g, depths_b);
+    else launch_bwd_channels<false>(ws, v, lane, s, io, sigma, flags, g, depths_b);
 }

@@ -30,15 +30,16 @@ struct DevEnv {
 template <int MAXC>
 static __device__ __forceinline__ void interior_adjoint_warp(const SceneView &s, int x, int y, bool has,
                                                              const PixelState<MAXC> &p, const float *g,
-                                                             const DeodrGrads &grads) {
+                                                             const DeodrGrads &grads, float *depths_b = nullptr) {
     const int lane = (int)(threadIdx.x & 31), C = s.nb_colors;
     TriAttr t;
     VertexGrads<MAXC> acc;
     zero_vertex_grads<MAXC>(s, &acc);
+    float dz[3] = {0.0f, 0.0f, 0.0f};  // depths_b (perspective_correct only)
     t.textured = false;
     if (has) {
         tri_attr(s, p.bown & TRI_INDEX_MASK, &t);
-        pixel_adjoint<MAXC, DevEnv>(s, t, x, y, g, &acc, grads.texture_b);
+        pixel_adjoint<MAXC, DevEnv>(s, t, x, y, g, &acc, grads.texture_b, dz);
     }
     const int key = has ? (p.bown & TRI_INDEX_MASK) : -1 - lane;  // idle lanes: groups of one
     const unsigned peers = __match_any_sync(0xffffffffu, key);
@@ -60,6 +61,10 @@ static __device__ __forceinline__ void interior_adjoint_warp(const SceneView &s,
             DEODR_TAKE(acc.ij[i][0]);
             DEODR_TAKE(acc.ij[i][1]);
         }
+        if (s.perspective_correct) {
+#pragma unroll
+            for (int i = 0; i < 3; i++) DEODR_TAKE(dz[i]);
+        }
         if (any_textured) {
 #pragma unroll
             for (int i = 0; i < 3; i++) {
@@ -79,7 +84,7 @@ static __device__ __forceinline__ void interior_adjoint_warp(const SceneView &s,
     }
     if (has && rank == 0)
         flush_vertex_grads<MAXC, AtomicEmit<DevEnv>>(s, t, acc, grads.ij_b, grads.colors_b, grads.uv_b, grads.shade_b,
-                                                     AtomicEmit<DevEnv>());
+                                                     AtomicEmit<DevEnv>(), dz, depths_b);
 }
 
 // The <1> and <3> instances are only launched for exactly 1 / 3 colour channels: telling the compiler turns every
@@ -224,5 +229,8 @@ static EdgeTiles edge_tiles_of(const ViewSlot *v) {
 
 
 // kernels_bwd.cu: enqueues the adjoint pass of one view on the lane's streams
+// rows of one edge's fp64 accumulators in the adjoint of view s (edge_acc_stride / edge_acc_stride_persp)
+int deodr_edge_acc_stride(const SceneView &s);
+// (depths_b: [V] fp32 of the view or NULL; only the perspective-correct instances write it)
 void deodr_launch_backward(DeodrWorkspace *ws, ViewSlot *v, Lane &lane, const SceneView &s, const DeodrViewIO &io,
-                           double sigma, int flags, const DeodrGrads &g);
+                           double sigma, int flags, const DeodrGrads &g, float *depths_b);

@@ -716,7 +716,7 @@ DEODR_HD void phase_edge_replay(const SceneView &s, int x, int y, int r, int n, 
     const int C = s.nb_colors;
     for (unsigned long long mask = edge_hit_mask(sh, n, r, x); mask; mask &= mask - 1) {
         const EdgeRec &rec = sh->edge.rec[lowest_bit64(mask)];
-        double ze = edge_z(rec, x, y, false);
+        double ze = edge_z(rec, x, y, s.perspective_correct != 0);
         if (!(ze < p.z)) continue;
         if (!a->has_colour) {
             PixelState<MAXC> q = p;
@@ -736,12 +736,12 @@ template <int MAXC, class Env>
 DEODR_HD void phase_edge_adjoint(const SceneView &s, int x, int y, int r, int n, const TileShared *sh,
                                  const PixelState<MAXC> &p, AdjointState<MAXC> *a, double *edge_acc, float *texture_b) {
     const int C = s.nb_colors;
-    const int stride = edge_acc_stride(C);
+    const int stride = s.perspective_correct ? edge_acc_stride_persp(C) : edge_acc_stride(C);
     for (unsigned long long mask = edge_hit_mask(sh, n, r, x); mask;) {  // near to far: highest bit first
         const int e = highest_bit64(mask);
         mask &= ~(1ull << e);
         const EdgeRec &rec = sh->edge.rec[e];
-        double ze = edge_z(rec, x, y, false);
+        double ze = edge_z(rec, x, y, s.perspective_correct != 0);
         if (!(ze < p.z)) continue;
         EdgeHit<MAXC> h;
         edge_hit<MAXC>(s, rec, x, y, ze, &h);
@@ -749,7 +749,64 @@ DEODR_HD void phase_edge_adjoint(const SceneView &s, int x, int y, int r, int n,
         const double T = h.T, omT = 1.0 - h.T;
         double T_B = 0;
         const double t3[3] = {(double)x, (double)y, 1.0};
-        if (s.texture != nullptr && rec.textured) {
+        if (s.perspective_correct) {
+            // the edge's attribute a = w_0 a_0 + w_1 a_1, w_q = b_q q_q Ze: the same adjoint as pixel_adjoint_persp
+            // over the two end points (edge_acc_stride_persp gives the layout)
+            const double w[2] = {h.b[0] * rec.inv_z[0] * ze, h.b[1] * rec.inv_z[1] * ze};
+            double sd[2] = {0.0, 0.0};
+            if (s.texture != nullptr && rec.textured) {
+                double L_B = 0;
+                float e0_B = 0, e1_B = 0;
+                for (int c = 0; c < C; c++) {
+                    double gc = (double)a->g[c];
+                    double prev = (a->col[c] - omT * (double)h.A[c]) / T;
+                    T_B += gc * (prev - (double)h.A[c]);
+                    a->col[c] = prev;
+                    float A_B = (float)(omT * gc) * h.L;
+                    L_B += omT * gc * (double)h.texval[c];
+                    texture_fetch_duv(h.tap, s.texture, c, A_B, &e0_B, &e1_B);
+                    if (texture_b) {
+                        float w00 = (1.0f - h.tap.e0) * (1.0f - h.tap.e1), w10 = h.tap.e0 * (1.0f - h.tap.e1);
+                        float w01 = (1.0f - h.tap.e0) * h.tap.e1, w11 = h.tap.e0 * h.tap.e1;
+                        Env::atomic_add(texture_b + h.tap.i00 + c, w00 * A_B);
+                        Env::atomic_add(texture_b + h.tap.i10 + c, w10 * A_B);
+                        Env::atomic_add(texture_b + h.tap.i01 + c, w01 * A_B);
+                        Env::atomic_add(texture_b + h.tap.i11 + c, w11 * A_B);
+                    }
+                    a->g[c] = (float)(gc * T);
+                }
+                const double U_B = h.tap.out0 ? 0.0 : (double)e0_B, V_B = h.tap.out1 ? 0.0 : (double)e1_B;
+                const double L = w[0] * (double)s.shade[rec.vid[0]] + w[1] * (double)s.shade[rec.vid[1]];
+                for (int q = 0; q < 2; q++) {
+                    const double uq = s.uv[2 * (size_t)rec.uvid[q]], vq = s.uv[2 * (size_t)rec.uvid[q] + 1];
+                    sd[q] = U_B * (uq - h.u) + V_B * (vq - h.v) + L_B * ((double)s.shade[rec.vid[q]] - L);
+                    Env::atomic_add(acc + 11 + 3 * q, w[q] * U_B);
+                    Env::atomic_add(acc + 12 + 3 * q, w[q] * V_B);
+                    Env::atomic_add(acc + 13 + 3 * q, w[q] * L_B);
+                }
+            } else {
+                for (int c = 0; c < C; c++) {
+                    double gc = (double)a->g[c];
+                    double prev = (a->col[c] - omT * (double)h.A[c]) / T;
+                    T_B += gc * (prev - (double)h.A[c]);
+                    a->col[c] = prev;
+                    const double A_B = omT * gc;
+                    const double a0 = (double)s.colors[(size_t)rec.vid[0] * C + c],
+                                 a1 = (double)s.colors[(size_t)rec.vid[1] * C + c];
+                    const double A = w[0] * a0 + w[1] * a1;
+                    sd[0] += A_B * (a0 - A);
+                    sd[1] += A_B * (a1 - A);
+                    Env::atomic_add(acc + 11 + c, w[0] * A_B);
+                    Env::atomic_add(acc + 11 + C + c, w[1] * A_B);
+                    a->g[c] = (float)(gc * T);
+                }
+            }
+            for (int q = 0; q < 2; q++) {
+                const double bq_B = rec.inv_z[q] * ze * sd[q];
+                for (int j = 0; j < 3; j++) Env::atomic_add(acc + 3 + 3 * q + j, bq_B * t3[j]);
+                Env::atomic_add(acc + 9 + q, -w[q] * sd[q] * rec.inv_z[q]);
+            }
+        } else if (s.texture != nullptr && rec.textured) {
             double L_B = 0;
             float e0_B = 0, e1_B = 0;
             for (int c = 0; c < C; c++) {
@@ -936,13 +993,14 @@ DEODR_HD void residual_adjoint(const SceneView &s, const float *col, const float
 template <int MAXC, class Env>
 DEODR_HD void phase_interior_adjoint(const SceneView &s, int x, int y, const PixelState<MAXC> &p, const float *g,
                                      float *ij_b, float *colors_b, float *uv_b, float *shade_b, float *texture_b,
-                                     const Env &env) {
+                                     const Env &env, float *depths_b = nullptr) {
     TriAttr t;
     tri_attr(s, p.bown & TRI_INDEX_MASK, &t);
     VertexGrads<MAXC> acc;
     zero_vertex_grads<MAXC>(s, &acc);
-    pixel_adjoint<MAXC, Env>(s, t, x, y, g, &acc, texture_b);
-    flush_vertex_grads<MAXC, Env>(s, t, acc, ij_b, colors_b, uv_b, shade_b, env);
+    float dz[3] = {0.0f, 0.0f, 0.0f};
+    pixel_adjoint<MAXC, Env>(s, t, x, y, g, &acc, texture_b, dz);
+    flush_vertex_grads<MAXC, Env>(s, t, acc, ij_b, colors_b, uv_b, shade_b, env, dz, depths_b);
 }
 
 // Plain atomics for the triangle-parallel adjoint.
@@ -959,7 +1017,8 @@ struct AtomicEmit {
 template <int MAXC, class Env>
 DEODR_HD void small_triangle_adjoint(const SceneView &s, int k, int tiles_x, const int *edge_tile_count,
                                      const int *owner, const int *tie_pairs, const float *image_b, float *ij_b,
-                                     float *colors_b, float *uv_b, float *shade_b, float *texture_b) {
+                                     float *colors_b, float *uv_b, float *shade_b, float *texture_b,
+                                     float *depths_b = nullptr) {
     const int C = s.nb_colors;
     double V[3][2];
     for (int i = 0; i < 3; i++) {
@@ -1017,9 +1076,11 @@ DEODR_HD void small_triangle_adjoint(const SceneView &s, int k, int tiles_x, con
     }
     // The two kinds of triangle keep different accumulators (vertex colours vs uv + shade): separate loops, so that the
     // common interpolated case holds 15 running sums in registers instead of a 24-float structure in local memory.
-    if (t.textured) {
+    // Perspective-correct triangles take the general loop (pixel_adjoint_persp).
+    if (t.textured || s.perspective_correct) {
         VertexGrads<MAXC> acc;
         zero_vertex_grads<MAXC>(s, &acc);
+        float dz[3] = {0.0f, 0.0f, 0.0f};
         for (;;) {
             const int i = i_next;
             float g[MAXC];
@@ -1031,10 +1092,11 @@ DEODR_HD void small_triangle_adjoint(const SceneView &s, int k, int tiles_x, con
                 const size_t idx = (size_t)(y0 + (i_next >> shift)) * s.width + x0 + (i_next & stride_mask);
                 for (int q = 0; q < C; q++) g_next[q] = image_b[idx * C + q];
             }
-            pixel_adjoint<MAXC, Env>(s, t, x0 + (i & stride_mask), y0 + (i >> shift), g, &acc, texture_b);
+            pixel_adjoint<MAXC, Env>(s, t, x0 + (i & stride_mask), y0 + (i >> shift), g, &acc, texture_b, dz);
             if (!more) break;
         }
-        flush_vertex_grads<MAXC, AtomicEmit<Env>>(s, t, acc, ij_b, colors_b, uv_b, shade_b, AtomicEmit<Env>());
+        flush_vertex_grads<MAXC, AtomicEmit<Env>>(s, t, acc, ij_b, colors_b, uv_b, shade_b, AtomicEmit<Env>(), dz,
+                                                  depths_b);
         return;
     }
     // interpolated triangle: per-triangle constants = vertex colours' screen-space gradient
@@ -1215,7 +1277,7 @@ DEODR_HD void small_record_adjoint(const SceneView &s, const PreRec &r, Tile til
 // DR.h:1758-1773 / 2045-2060 followed by get_edge_stencil_equations_B DR.h:1462-1539.
 template <class Env>
 DEODR_HD void finalize_edge(const SceneView &s, int edge_id, double sigma, const double *acc, float *ij_b,
-                            float *colors_b, float *uv_b, float *shade_b) {
+                            float *colors_b, float *uv_b, float *shade_b, float *depths_b = nullptr) {
     const int C = s.nb_colors;
     int k = edge_id / 3, n = edge_id - 3 * k;
     uint32_t vid[2], uvid[2];
@@ -1235,7 +1297,19 @@ DEODR_HD void finalize_edge(const SceneView &s, int edge_id, double sigma, const
     const bool textured = s.textured[k] && s.shaded[k];
     double Einv_B[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     for (int j = 0; j < 3; j++) Einv_B[6 + j] += acc[j] * (1.0 / sigma);  // T = (row 2 of Einv) / sigma
-    if (textured) {
+    if (s.perspective_correct) {  // layout of edge_acc_stride_persp: b_q = (row q of Einv) . (x, y, 1)
+        for (int q = 0; q < 2; q++) {
+            for (int j = 0; j < 3; j++) Einv_B[3 * q + j] += acc[3 + 3 * q + j];
+            if (depths_b) Env::atomic_add(depths_b + vid[q], (float)acc[9 + q]);
+            if (textured) {
+                Env::atomic_add(uv_b + 2 * (size_t)uvid[q], (float)acc[11 + 3 * q]);
+                Env::atomic_add(uv_b + 2 * (size_t)uvid[q] + 1, (float)acc[12 + 3 * q]);
+                Env::atomic_add(shade_b + vid[q], (float)acc[13 + 3 * q]);
+            } else {
+                for (int c = 0; c < C; c++) Env::atomic_add(colors_b + (size_t)vid[q] * C + c, (float)acc[11 + q * C + c]);
+            }
+        }
+    } else if (textured) {
         for (int q = 0; q < 2; q++) {  // edge vertex q
             double sh_b = 0, u_b = 0, v_b = 0;
             double shade_q = (double)s.shade[vid[q]];

@@ -255,8 +255,18 @@ DEODR_HD void zero_vertex_grads(const SceneView &s, VertexGrads<MAXC> *a) {
 //   attr_b[v]  += (d colour / d attr) g * b_v          ij_b[v][d] -= b_v * sum_c g_c * d colour_c / d x_d
 // accumulated into `acc`; texel adjoints go straight to texture_b (summed, see INTEGRATION.md).
 template <int MAXC, class Env>
+DEODR_HD void pixel_adjoint_persp(const SceneView &s, const TriAttr &t, int x, int y, const float *g,
+                                  VertexGrads<MAXC> *acc, float *depth_acc, float *texture_b);
+
+// (depth_acc: [3] running depths_b of the vertices, perspective_correct only; kept out of VertexGrads so that the
+// instances without perspective carry nothing more)
+template <int MAXC, class Env>
 DEODR_HD void pixel_adjoint(const SceneView &s, const TriAttr &t, int x, int y, const float *g, VertexGrads<MAXC> *acc,
-                            float *texture_b) {
+                            float *texture_b, float *depth_acc = nullptr) {
+    if (s.perspective_correct) {
+        pixel_adjoint_persp<MAXC, Env>(s, t, x, y, g, acc, depth_acc, texture_b);
+        return;
+    }
     const int C = s.nb_colors;
     PixelEval<MAXC> e;
     float colour[MAXC];
@@ -311,14 +321,91 @@ DEODR_HD void pixel_adjoint(const SceneView &s, const TriAttr &t, int x, int y, 
     }
 }
 
-// Scatter of one triangle's accumulated vertex gradients; `emit.emit(ptr, value)` adds value to *ptr.
+// Perspective-correct form of pixel_adjoint (DESIGN.md section 4).  With the plain barycentrics b_i, q_i = 1/z_i,
+// Z = 1 / sum_k b_k q_k and the weights w_i = b_i q_i Z, every attribute is a = sum_i w_i a_i, and for its adjoint a_B:
+//   a_i_B += w_i a_B      s_i = sum_attributes a_B (a_i - a)      b_i_B = q_i Z s_i      depths_b_i += -w_i s_i / z_i
+//   ij_b[v] -= b_v sum_j b_j_B grad b_j          (d b_j / d V_v = -b_v grad b_j: the PLAIN b_v, not w_v)
+// Z is recomputed from b and q (one fp64 reciprocal) rather than read from the z-buffer: every adjoint kernel can do
+// that, only the edge-tile kernel has the z-buffer at hand.  s_i and the screen-space sums are formed in fp64 (the
+// cancellation of pixel_adjoint).
+template <int MAXC, class Env>
+DEODR_HD void pixel_adjoint_persp(const SceneView &s, const TriAttr &t, int x, int y, const float *g,
+                                  VertexGrads<MAXC> *acc, float *depth_acc, float *texture_b) {
+    const int C = s.nb_colors;
+    const double px = (double)x - t.x0, py = (double)y - t.y0;
+    double b[3], w[3], sd[3] = {0.0, 0.0, 0.0};
+    b[1] = px * t.gx[1] + py * t.gy[1];
+    b[2] = px * t.gx[2] + py * t.gy[2];
+    b[0] = 1.0 - b[1] - b[2];
+    const double Z = 1.0 / (b[0] * t.inv_z[0] + b[1] * t.inv_z[1] + b[2] * t.inv_z[2]);
+    for (int i = 0; i < 3; i++) w[i] = b[i] * t.inv_z[i] * Z;
+    if (t.textured) {
+        double u = 0, v = 0, L = 0, ui[3], vi[3], li[3];
+        for (int i = 0; i < 3; i++) {
+            ui[i] = s.uv[2 * (size_t)t.uvid[i]];
+            vi[i] = s.uv[2 * (size_t)t.uvid[i] + 1];
+            li[i] = (double)s.shade[t.vid[i]];
+            u += w[i] * ui[i];
+            v += w[i] * vi[i];
+            L += w[i] * li[i];
+        }
+        const Tap tap = texture_tap(u, v, s.texture_width, s.texture_height, C);
+        float L_B = 0, e0_B = 0, e1_B = 0;
+        for (int c = 0; c < C; c++) {
+            const float A_B = g[c] * (float)L;
+            L_B += g[c] * texture_fetch(tap, s.texture, c);
+            texture_fetch_duv(tap, s.texture, c, A_B, &e0_B, &e1_B);
+            if (texture_b) {
+                float w00 = (1.0f - tap.e0) * (1.0f - tap.e1), w10 = tap.e0 * (1.0f - tap.e1);
+                float w01 = (1.0f - tap.e0) * tap.e1, w11 = tap.e0 * tap.e1;
+                Env::atomic_add(texture_b + tap.i00 + c, w00 * A_B);
+                Env::atomic_add(texture_b + tap.i10 + c, w10 * A_B);
+                Env::atomic_add(texture_b + tap.i01 + c, w01 * A_B);
+                Env::atomic_add(texture_b + tap.i11 + c, w11 * A_B);
+            }
+        }
+        const double U_B = tap.out0 ? 0.0 : (double)e0_B, V_B = tap.out1 ? 0.0 : (double)e1_B;
+        for (int i = 0; i < 3; i++) {
+            sd[i] = U_B * (ui[i] - u) + V_B * (vi[i] - v) + (double)L_B * (li[i] - L);
+            acc->uv[i][0] += (float)(U_B * w[i]);
+            acc->uv[i][1] += (float)(V_B * w[i]);
+            acc->shade[i] += (float)((double)L_B * w[i]);
+        }
+    } else {
+        for (int c = 0; c < C; c++) {
+            const double a0 = (double)s.colors[(size_t)t.vid[0] * C + c], a1 = (double)s.colors[(size_t)t.vid[1] * C + c],
+                         a2 = (double)s.colors[(size_t)t.vid[2] * C + c];
+            const double a = w[0] * a0 + w[1] * a1 + w[2] * a2, gc = (double)g[c];
+            sd[0] += gc * (a0 - a);
+            sd[1] += gc * (a1 - a);
+            sd[2] += gc * (a2 - a);
+            for (int i = 0; i < 3; i++) acc->attr[i][c] += (float)(gc * w[i]);
+        }
+    }
+    double dx = 0, dy = 0;  // sum_j b_j_B grad b_j
+    for (int j = 0; j < 3; j++) {
+        const double bj_B = t.inv_z[j] * Z * sd[j];
+        dx += bj_B * t.gx[j];
+        dy += bj_B * t.gy[j];
+        depth_acc[j] -= (float)(w[j] * sd[j] * t.inv_z[j]);
+    }
+    for (int i = 0; i < 3; i++) {
+        acc->ij[i][0] -= (float)(b[i] * dx);
+        acc->ij[i][1] -= (float)(b[i] * dy);
+    }
+}
+
+// Scatter of one triangle's accumulated vertex gradients; `emit.emit(ptr, value)` adds value to *ptr.  depths_b is only
+// written by the perspective-correct instances.
 template <int MAXC, class Emit>
 DEODR_HD void flush_vertex_grads(const SceneView &s, const TriAttr &t, const VertexGrads<MAXC> &acc, float *ij_b,
-                                 float *colors_b, float *uv_b, float *shade_b, const Emit &emit) {
+                                 float *colors_b, float *uv_b, float *shade_b, const Emit &emit,
+                                 const float *depth_acc = nullptr, float *depths_b = nullptr) {
     const int C = s.nb_colors;
     for (int i = 0; i < 3; i++) {
         emit.emit(ij_b + 2 * (size_t)t.vid[i], acc.ij[i][0]);
         emit.emit(ij_b + 2 * (size_t)t.vid[i] + 1, acc.ij[i][1]);
+        if (s.perspective_correct && depths_b) emit.emit(depths_b + t.vid[i], depth_acc[i]);
         if (t.textured) {
             emit.emit(uv_b + 2 * (size_t)t.uvid[i], acc.uv[i][0]);
             emit.emit(uv_b + 2 * (size_t)t.uvid[i] + 1, acc.uv[i][1]);
@@ -427,6 +514,14 @@ DEODR_HD void edge_hit(const SceneView &s, const EdgeRec &r, int x, int y, doubl
 //   [6..11]  UV_B     : sum UV_B[q] * (x, y, 1), q = 0, 1   (textured)
 //   [12..]   A_B      : sum A_B[c] * (x, y, 1), c < C       (interpolated)
 DEODR_HD int edge_acc_stride(int C) { return 12 + 3 * C; }
+
+// Layout of the same accumulators in the perspective-correct instances: the attribute weights w_i = b_i q_i Ze are not
+// planes over (x, y, 1) any more, so the rows hold the adjoints of the two barycentric planes and per-end-point sums.
+//   [0..2]   transp_B : sum T_B * (x, y, 1)
+//   [3..8]   b_B      : sum b_q_B * (x, y, 1), q = 0, 1
+//   [9..10]  depths_b : sum -w_q s_q / z_q, q = 0, 1
+//   [11..]   a_B      : sum w_q a_B: colours [q * C + c] (interpolated) or (u, v, L) [3 q + 0..2] (textured)
+DEODR_HD int edge_acc_stride_persp(int C) { return 11 + (2 * C > 6 ? 2 * C : 6); }
 
 // Adjoint of inv3x3 (DR.h:124-232): S_B += d(inv)/dS^T T_B, with Tinv = inv(S):  S_B = -Tinv^T T_B Tinv^T.
 DEODR_HD void inv3x3_adjoint(const double *Tinv, const double *T_B, double *S_B) {

@@ -241,11 +241,14 @@ class DeviceMeshView:
         -> luminosity / normals / projection adjoints -> vertices_b (+ vertex_colors_b, light_b)
 
     No tensor crosses PCIe inside :meth:`render` / :meth:`backward`; the shared gradients of several views are plain
-    CUDA tensors that a caller sums over views and all-reduces over ranks (deodr_b200.distributed)."""
+    CUDA tensors that a caller sums over views and all-reduces over ranks (deodr_b200.distributed).
+
+    ``perspective_correct=True`` renders with perspective-correct interpolation; :meth:`backward` then also takes the
+    rasteriser's gradient of the vertex depths through the projection adjoint."""
 
     def __init__(self, faces, nb_vertices: int, camera: CameraParams, height: int, width: int, renderer=None,
                  light_directional=None, ambient: float = 1.0, background_color=(0.0, 0.0, 0.0), sigma: float = 1.0,
-                 clockwise: bool = False, device="cuda", slot: int = 0):
+                 clockwise: bool = False, device="cuda", slot: int = 0, perspective_correct: bool = False):
         from .renderer import DeviceScene, default_renderer
         from .scenes import SceneArrays
 
@@ -262,7 +265,7 @@ class DeviceMeshView:
             shaded=np.zeros(T, bool), edgeflags=np.zeros((T, 3), bool), height=height, width=width, nb_colors=nb_colors,
             texture=np.zeros((2, 2, nb_colors)), background_image=None,
             background_color=np.asarray(background_color, dtype=np.float64), clockwise=clockwise, backface_culling=True,
-            strict_edge=True, perspective_correct=False, integer_pixel_centers=True)
+            strict_edge=True, perspective_correct=bool(perspective_correct), integer_pixel_centers=True)
         self.scene = DeviceScene(arrays, self.device)
         self.renderer = renderer if renderer is not None else default_renderer(self.device.index)
         self._saved = None
@@ -284,10 +287,12 @@ class DeviceMeshView:
     def backward(self, image_b: torch.Tensor, reference_transpose: bool = False) -> Dict[str, torch.Tensor]:
         """-> dict(vertices_b [V,3] f64, vertex_colors_b [V,C] f64, light_b [4] f64)."""
         vertices, vertex_colors, normals, fwd = self._saved
-        grads = self.renderer.render_b(self.scene, self.sigma, fwd, image_b)
+        persp = self.scene.perspective_correct
+        grads = self.renderer.render_b(self.scene, self.sigma, fwd, image_b, depths_b=persp)
         lum = vertex_luminosity_backward(normals, vertex_colors, self.light_directional, self.ambient,
                                          colors_b=grads["colors_b"])
         vertices_b = self.topology.vertex_normals_backward(vertices, lum["normals_b"])
-        project_points_backward(vertices, self.camera, grads["ij_b"], out=vertices_b,
+        project_points_backward(vertices, self.camera, grads["ij_b"],
+                                depths_b=grads["depths_b"].to(torch.float64) if persp else None, out=vertices_b,
                                 reference_transpose=reference_transpose)
         return {"vertices_b": vertices_b, "vertex_colors_b": lum["vertex_colors_b"], "light_b": lum["light_b"]}

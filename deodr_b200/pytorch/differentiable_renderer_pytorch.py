@@ -11,7 +11,7 @@ Two Functions with the reference contract ``(ij, colors, scene) -> image[H,W,C]`
 
 from __future__ import annotations
 
-from typing import Any
+from typing import Any, Optional
 
 import numpy as np
 import torch
@@ -55,19 +55,26 @@ TorchDifferentiableRender2D = TorchDifferentiableRenderer2DFunc.apply
 
 
 class CudaDifferentiableRenderer2DFunc(torch.autograd.Function):
-    """Device-resident variant: ``image = f(ij[V,2] f64 cuda, colors[V,C] cuda, DeviceScene, sigma)``.
+    """Device-resident variant: ``image = f(ij[V,2] f64 cuda, colors[V,C] cuda, DeviceScene, sigma[, depths[V]])``.
+
+    ``depths`` (optional) is written into the scene and receives a gradient: with a ``perspective_correct`` scene the
+    image depends on the vertex depths (zero gradient otherwise).
 
     The renderer keeps ONE live forward state per slot, and the ``DeviceScene`` is shared and mutable, so the node
     snapshots its inputs; if another forward has used the slot by the time ``backward`` runs (two renders before
     ``loss.backward()``), the forward is replayed from the snapshot first."""
 
     @staticmethod
-    def forward(ctx: Any, ij: torch.Tensor, colors: torch.Tensor, scene: DeviceScene, sigma: float = 1.0):  # type: ignore
-        scene.update(ij=ij.detach(), colors=colors.detach())
+    def forward(ctx: Any, ij: torch.Tensor, colors: torch.Tensor, scene: DeviceScene, sigma: float = 1.0,  # type: ignore
+                depths: Optional[torch.Tensor] = None):
+        arrays = {"ij": ij.detach(), "colors": colors.detach()}
+        if depths is not None:
+            arrays["depths"] = depths.detach()
+        scene.update(**arrays)
         fwd = default_renderer(scene.device.index).render(scene, sigma)
         ctx.scene, ctx.sigma, ctx.fwd = scene, float(sigma), fwd
-        ctx.in_dtypes = (ij.dtype, colors.dtype)
-        ctx.save_for_backward(ij.detach().clone(), colors.detach().clone())
+        ctx.in_dtypes = (ij.dtype, colors.dtype, depths.dtype if depths is not None else None)
+        ctx.save_for_backward(*[a.clone() for a in arrays.values()])
         # the caller gets its own tensor: the framebuffers of ctx.fwd may be re-rendered into by backward
         return fwd["image"].clone()
 
@@ -75,14 +82,17 @@ class CudaDifferentiableRenderer2DFunc(torch.autograd.Function):
     def backward(ctx: Any, *grad_outputs: Any) -> Any:
         (image_b,) = grad_outputs
         renderer = default_renderer(ctx.scene.device.index)
-        ij, colors = ctx.saved_tensors
+        saved = ctx.saved_tensors
+        arrays = dict(zip(("ij", "colors", "depths"), saved))
+        with_depths = len(saved) == 3
         if ctx.fwd["generation"] != renderer.generation(ctx.fwd["slot"]):
-            ctx.scene.update(ij=ij, colors=colors)
+            ctx.scene.update(**arrays)
             ctx.fwd = renderer.render(ctx.scene, ctx.sigma, out=ctx.fwd)
         else:
-            ctx.scene.update(ij=ij, colors=colors)  # the shared scene may hold another node's inputs by now
-        grads = renderer.render_b(ctx.scene, ctx.sigma, ctx.fwd, image_b)
-        return grads["ij_b"].to(ctx.in_dtypes[0]), grads["colors_b"].to(ctx.in_dtypes[1]), None, None
+            ctx.scene.update(**arrays)  # the shared scene may hold another node's inputs by now
+        grads = renderer.render_b(ctx.scene, ctx.sigma, ctx.fwd, image_b, depths_b=with_depths)
+        depths_b = grads["depths_b"].to(ctx.in_dtypes[2]) if with_depths else None
+        return grads["ij_b"].to(ctx.in_dtypes[0]), grads["colors_b"].to(ctx.in_dtypes[1]), None, None, depths_b
 
 
 CudaDifferentiableRender2D = CudaDifferentiableRenderer2DFunc.apply

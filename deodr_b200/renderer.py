@@ -225,13 +225,13 @@ class Renderer:
 
     def render_b(self, scene: DeviceScene, sigma: float, fwd: dict, image_b: Optional[torch.Tensor] = None,
                  grads: Optional[Dict[str, torch.Tensor]] = None, err_buffer_b: Optional[torch.Tensor] = None,
-                 error_adjoint_complete: bool = False) -> Dict[str, torch.Tensor]:
+                 error_adjoint_complete: bool = False, depths_b: bool = False) -> Dict[str, torch.Tensor]:
         """Adjoint pass; accumulates into ``grads`` (created zeroed if None) and returns it.  In antialiase_error mode
-        pass ``err_buffer_b`` ([H,W]) instead of ``image_b``."""
+        pass ``err_buffer_b`` ([H,W]) instead of ``image_b``.  ``depths_b=True``: see :meth:`render_b_views`."""
         return self.render_b_views([scene], sigma, [fwd], [image_b] if image_b is not None else None,
                                    [grads] if grads is not None else None,
                                    [err_buffer_b] if err_buffer_b is not None else None,
-                                   error_adjoint_complete=error_adjoint_complete)[0]
+                                   error_adjoint_complete=error_adjoint_complete, depths_b=depths_b)[0]
 
     # ---- batch of views (slots 0 .. n-1) --------------------------------------------------------------------------
     def render_views(self, scenes: Sequence[DeviceScene], sigma: float, face_id: bool = False,
@@ -271,13 +271,21 @@ class Renderer:
                        image_bs: Optional[Sequence[torch.Tensor]] = None,
                        grads: Optional[Sequence[Dict[str, torch.Tensor]]] = None,
                        err_buffer_bs: Optional[Sequence[torch.Tensor]] = None,
-                       error_adjoint_complete: bool = False) -> List[Dict[str, torch.Tensor]]:
+                       error_adjoint_complete: bool = False, depths_b: bool = False) -> List[Dict[str, torch.Tensor]]:
         """Adjoint passes of the views rendered by :meth:`render_views` (same order).  Entries of ``grads`` may share
-        tensors: gradients of shared parameters accumulate in place (the ``+=`` of deodr/mesh_fitter.py:518-527)."""
+        tensors: gradients of shared parameters accumulate in place (the ``+=`` of deodr/mesh_fitter.py:518-527).
+
+        ``depths_b=True`` goes through deodr_b200_render_b_views_depths: ``perspective_correct`` views are accepted and
+        each view's dict gets (or accumulates into its own) ``"depths_b"`` [V] fp32, the gradient of the vertex depths.
+        It stays zero for views without ``perspective_correct``, whose image does not depend on the depths."""
         n = len(scenes)
         err_mode = err_buffer_bs is not None
         if grads is None:
             grads = [s.zero_grads() for s in scenes]
+        if depths_b:
+            for s, g in zip(scenes, grads):
+                if g.get("depths_b") is None:
+                    g["depths_b"] = torch.zeros(s.t["depths"].shape, dtype=torch.float32, device=s.device)
         for i, f in enumerate(fwds):
             if f.get("generation") is not None and f["generation"] != self.generation(f.get("slot", i)):
                 raise RuntimeError(
@@ -301,8 +309,13 @@ class Renderer:
                           for k in ("ij_b", "colors_b", "uv_b", "shade_b", "texture_b"))) for g in grads])
         flags = (_cabi.ANTIALIASE_ERROR if err_mode else 0) | (_cabi.ERROR_ADJOINT_COMPLETE if error_adjoint_complete else 0)
         with self._lock:
-            _cabi.check(self.lib.deodr_b200_render_b_views(self._ws, n, views, (_cabi.ViewIO * n)(*ios), gs,
-                                                           float(sigma), flags, self._stream()))
+            if depths_b:
+                dbs = (C.c_void_p * n)(*[g["depths_b"].data_ptr() if g["depths_b"].numel() > 0 else None for g in grads])
+                _cabi.check(self.lib.deodr_b200_render_b_views_depths(self._ws, n, views, (_cabi.ViewIO * n)(*ios), gs,
+                                                                      dbs, float(sigma), flags, self._stream()))
+            else:
+                _cabi.check(self.lib.deodr_b200_render_b_views(self._ws, n, views, (_cabi.ViewIO * n)(*ios), gs,
+                                                               float(sigma), flags, self._stream()))
         del keep
         return list(grads)
 

@@ -34,7 +34,9 @@ extern "C" {
 enum {
     DEODR_B200_OK = 0,
     DEODR_B200_EINVAL = 1,      /* null pointer / bad size / index out of range (checkSceneValid, DR.h:2664) */
-    DEODR_B200_EUNSUPPORTED = 2,/* backward with perspective_correct or without backface_culling (DR.h:810, 2924) */
+    DEODR_B200_EUNSUPPORTED = 2,/* backward without backface_culling (DR.h:2924); backward with perspective_correct
+                                   through any adjoint entry point but deodr_b200_render_b_views_depths (DR.h:810),
+                                   and there together with antialiase_error */
     DEODR_B200_ECUDA = 3,       /* CUDA runtime failure */
     DEODR_B200_ENOMEM = 4,
     DEODR_B200_EREPLAN = 5      /* deferred mode only: a forward overflowed the lists its plan had reserved; the
@@ -189,6 +191,16 @@ int deodr_b200_render_views(DeodrWorkspace *ws, int n_views, const DeodrSceneVie
  * gets its own ij_b. */
 int deodr_b200_render_b_views(DeodrWorkspace *ws, int n_views, const DeodrSceneView *views, const DeodrViewIO *io,
                               const DeodrGrads *grads, double sigma, int flags, void *stream);
+
+/* Adjoint passes of the views, as deodr_b200_render_b_views, that also accept perspective_correct scenes and return
+ * the gradient of the vertex depths: depths_b[i] is a device pointer to [V] fp32 of view i (or NULL), accumulated
+ * into.  For views without perspective_correct the depths do not reach the image and depths_b[i] is left untouched.
+ * With perspective_correct the interpolation weights depend on the depths; the z-buffer test only decides which
+ * triangle or edge owns a pixel and has no adjoint.  DEODR_B200_ANTIALIASE_ERROR together with a perspective_correct
+ * view is refused (DEODR_B200_EUNSUPPORTED). */
+int deodr_b200_render_b_views_depths(DeodrWorkspace *ws, int n_views, const DeodrSceneView *views,
+                                     const DeodrViewIO *io, const DeodrGrads *grads, float *const *depths_b,
+                                     double sigma, int flags, void *stream);
 
 /* Deferred mode (on = 1): the entry points never read the verdict themselves - nothing in them touches the host side
  * of the device, so a forward + adjoint sequence can be captured in a CUDA graph (they also behave this way whenever

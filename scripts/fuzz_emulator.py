@@ -22,6 +22,10 @@ canvases up to 270 x 270 (DEODR_FUZZ_SCALE=3), 3.7 million with the exact-wrap b
 perspective_correct at 3-4e-4 relative image error (fp32 attributes of triangles 1e9 px long).  What the campaigns did
 find: a pixel owned by a visible sliver judged without its weight scale in error mode (criterion fixed), a first row
 of 32768 in the exact-wrap build (fixed), and the reference itself corrupting its heap beyond its `short` range.
+Scenes drawn with perspective_correct (one in four) check their adjoint through emul_render_b_depths against the port
+oracle's perspective-correct adjoint (tests/perspective_support.py; the compiled reference has none), depths_b included,
+under the same
+gradient criterion: 417 thousand scenes over five seeds, 83,484 of them perspective-correct adjoints, no failure.
 """
 import os
 import sys
@@ -32,8 +36,8 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-from canon import Emulator  # noqa: E402
 from oracle.oracle import Oracle  # noqa: E402
+from perspective_support import PerspEmulator, PerspOracle  # noqa: E402
 
 from deodr_b200.scenes import confetti_scene, dense_image_b, soup_scene, torus_scene  # noqa: E402
 
@@ -41,7 +45,9 @@ tex = np.load(os.path.join(ROOT, "tests/golden/trefle_texture_u8.npy")).astype(n
 # DEODR_FUZZ_EXACT_WRAP=1: the emulation built with DEODR_EXACT_SHORT_WRAP=1 (rmath.h), and one scene in three gets a few
 # vertices pushed 4e4 .. 1e9 pixels away (beyond the reference's `short` range: only that build follows the reference there)
 EXACT_WRAP = os.environ.get("DEODR_FUZZ_EXACT_WRAP", "0") == "1"
-emu, ora = Emulator(exact_short_wrap=EXACT_WRAP), Oracle("reference", texfix=True)
+ora = Oracle("reference", texfix=True)
+emu = PerspEmulator(exact_short_wrap=EXACT_WRAP)  # the emulation, with emul_render_b_depths
+port = PerspOracle(texfix=True)  # the perspective-correct adjoint (render_b_depths)
 rng_far = np.random.default_rng(12345 + (int(sys.argv[1]) if len(sys.argv) > 1 else 0))
 rng = np.random.default_rng(int(sys.argv[1]) if len(sys.argv) > 1 else 0)
 limit = float(sys.argv[2]) if len(sys.argv) > 2 else 300.0
@@ -49,7 +55,7 @@ only = int(sys.argv[3]) if len(sys.argv) > 3 else 0  # replay: generate every sc
 # DEODR_FUZZ_SCALE=3: canvases up to 270 x 270 (17 x 17 tiles: more tiles per triangle, longer per-tile lists, more
 # triangles and edges per scene); the default keeps the scenes of the earlier campaigns (same random streams)
 SCALE = float(os.environ.get("DEODR_FUZZ_SCALE", "1"))
-t0, n, bad, special = time.time(), 0, 0, 0
+t0, n, bad, special, n_persp_b = time.time(), 0, 0, 0, 0
 worst = {"image": 0.0, "grad": 0.0}
 while time.time() - t0 < limit and (only == 0 or n < only):
     kind = int(rng.integers(0, 4))
@@ -171,11 +177,18 @@ while time.time() - t0 < limit and (only == 0 or n < only):
     # observed up to 7.3e-5 over 30 000 such scenes)
     if err > (2.5e-4 if far_scene else 6e-5):
         msg += f" image {err:.2e}"
-    if scene.backface_culling and not scene.perspective_correct:
+    if scene.backface_culling:
         image_b = dense_image_b(image)
-        ref = ora.render_b(scene, sigma, image, z, image_b)
-        got = emu.render_b(scene, sigma, fwd, image_b)
-        for name in ("ij_b", "colors_b", "uv_b", "shade_b", "texture_b"):
+        names = ("ij_b", "colors_b", "uv_b", "shade_b", "texture_b")
+        if scene.perspective_correct:
+            n_persp_b += 1
+            ref = port.render_b_depths(scene, sigma, image, z, image_b)
+            got = emu.render_b_depths(scene, sigma, fwd, image_b)
+            names += ("depths_b",)
+        else:
+            ref = ora.render_b(scene, sigma, image, z, image_b)
+            got = emu.render_b(scene, sigma, fwd, image_b)
+        for name in names:
             if ref[name].size == 0:
                 continue
             m, d = np.abs(ref[name]).max(), np.abs(got[name] - ref[name]).max()
@@ -191,5 +204,6 @@ while time.time() - t0 < limit and (only == 0 or n < only):
         print("FAIL scene", n, "kind", kind, (W, H), "T", scene.faces.shape[0], "sigma", sigma, "strict", scene.strict_edge,
               "half-pixel centres", not scene.integer_pixel_centers, "cull", scene.backface_culling, "persp",
               scene.perspective_correct, msg, flush=True)
-print(f"{n} scenes, {bad} failures, {special} measure-zero cases outside the generic tolerance; worst relative image "
-      f"error {worst['image']:.2e}, worst relative gradient error (generic position) {worst['grad']:.2e}")
+print(f"{n} scenes ({n_persp_b} perspective-correct adjoints), {bad} failures, {special} measure-zero cases outside the "
+      f"generic tolerance; worst relative image error {worst['image']:.2e}, worst relative gradient error (generic "
+      f"position) {worst['grad']:.2e}")
